@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]          # uav_b200 arm (N>1: launched by torch.distributed.run)
     python bench.py --impl reference [--gpus N] ...              # reference arm: the path's own CPU implementation
+    python bench.py ... --dump-outputs DIR                       # also write the last timed step's frames to DIR/*.npy
 
 One "step" = one full pass of the hot path over one synthetic clip: `VideoUpscalePipeline.__call__` with 30 DDIM
 steps (chunked UNet, CFG, step_v0, flow propagation at steps 24/26/28, step_vt) followed by the chunked VAE decode.
@@ -356,6 +357,23 @@ def reference_gpu_leg(device, h_image, h_fw, h_bw, pe, steps, prop):
         torch.backends.cudnn.benchmark = bench_flag
 
 
+DUMP_SAMPLES = 1 << 23   # values kept per dumped output: 32 MB of float32
+
+
+def dump_outputs(dirname, outputs):
+    """Write each output tensor to `dirname/<name>.npy` as float32, so that two builds run with the same arguments can be
+    compared value for value.  An output of more than DUMP_SAMPLES values is stored as the values at DUMP_SAMPLES flat
+    positions drawn with a fixed seed and sorted: the same positions for the same shape, on every run."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in outputs.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLES:
+            idx = torch.randint(t.numel(), (DUMP_SAMPLES,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(dirname, f"{name}.npy"), t.float().cpu().numpy())
+
+
 _REAL_STDOUT = None
 
 
@@ -398,7 +416,11 @@ def main():
     ap.add_argument("--no-reference-gpu", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--no-e2e", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--warmup-ddim-steps", type=int, default=0, help=argparse.SUPPRESS)  # side configs: cheap warm-up clips
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned to DIR/<name>.npy (float32; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     t_start = time.time()
     _claim_stdout()
     if args.impl == "reference":
@@ -455,17 +477,18 @@ def main():
         torch.cuda.synchronize()
 
     def timed(fn, k):
+        """ms of k calls of fn, and what the last call returned"""
         barrier()
         s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s.record()
         for _ in range(k):
-            fn()
+            out = fn()
         e.record()
         barrier()
         ms = torch.tensor([s.elapsed_time(e)], device=device)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), out
 
     if args.warmup_ddim_steps:  # (hidden) warm the caches / packed weights with short clips; the timed clips are full length
         full = dict(kw)
@@ -480,15 +503,18 @@ def main():
         clocks.start()
     l0 = _lib.launch_count()
     sharding.comm_events_reset(True)
-    ms_total = timed(step_resident, args.steps)
+    ms_total, images = timed(step_resident, args.steps)
     comm_ms = sharding.comm_events_ms()
     sharding.comm_events_reset(False)
     launches = _lib.launch_count() - l0
-    # the end-to-end leg repeats whole clips (11 s each at config 2): at most E2E_MAX_STEPS of them, so that the driver's
-    # `--steps 20 --warmup 5` command (45 clips otherwise) stays well inside its per-run time limit
+    # the end-to-end leg repeats whole clips (11 s each at config 2): at most E2E_MAX_STEPS of them, so that a
+    # `--steps 20 --warmup 5` run (45 clips otherwise) stays under ten minutes
     e2e_steps = min(args.steps, E2E_MAX_STEPS)
-    ms_e2e = None if args.no_e2e else timed(step_e2e, e2e_steps)
+    ms_e2e = None if args.no_e2e else timed(step_e2e, e2e_steps)[0]
     clk = clocks.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"images": images})
+    del images
 
     # roofline of the dominant kernel (tcgen05 implicit GEMM): per-launch CUDA events over one UNet forward
     roof = None

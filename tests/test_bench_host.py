@@ -56,6 +56,22 @@ def test_host_threads_is_bounded():
     assert 1 <= n <= 32 and n <= (os.cpu_count() or 1)
 
 
+def test_dump_outputs_is_float32_bounded_and_reproducible(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    assert bench.DUMP_SAMPLES * 4 + 128 <= 64 << 20     # one float32 .npy (header included) per output, 64 MB in all
+    monkeypatch.setattr(bench, "DUMP_SAMPLES", 1000)
+    small = torch.randn(2, 3, 4, dtype=torch.float16)
+    big = torch.arange(5000, dtype=torch.float64).reshape(1, 5, 1000)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"small": small, "big": big})
+    a_small, a_big = np.load(tmp_path / "a" / "small.npy"), np.load(tmp_path / "a" / "big.npy")
+    assert a_small.dtype == np.float32 and a_small.shape == (2, 3, 4) and np.array_equal(a_small, small.float().numpy())
+    assert a_big.dtype == np.float32 and a_big.shape == (1000,)
+    assert np.all(np.diff(a_big) >= 0) and np.all(a_big == np.round(a_big))       # sorted positions of the flat output
+    assert np.array_equal(a_big, np.load(tmp_path / "b" / "big.npy"))            # same positions on every run
+
+
 def test_roofline_traffic_comes_from_the_committed_ncu_summary():
     prof = bench._ncu_profile_of_dominant_kernel()
     raw = json.load(open(os.path.join(ROOT, "profiles", "ncu_igemm_representative.json")))
